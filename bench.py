@@ -423,6 +423,7 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     ms = e0.elapsed_time(e1)
     launches = launches_now() - launches0
+    last_step = ff.results_to_host(out, out_ts, n_out) if args.dump_outputs else None  # (read after the clock stopped)
     results1 = ff.results_total()
     # per-phase device times (CUDA events inside the call) on PHASE_STEPS further steps, outside the timed region: the event records cost ~10 us per step
     for _ in range(2):
@@ -458,6 +459,14 @@ def run_ours(args):
     if pipe is not None:
         pipe.flush(out, out_ts, n_out)
         torch.cuda.synchronize()
+    if last_step is not None:
+        if world > 1:
+            gathered = [None] * world if rank == 0 else None
+            dist.gather_object(last_step, gathered, dst=0)
+            if rank == 0:
+                last_step = (np.concatenate([g[0] for g in gathered]), np.concatenate([g[1] for g in gathered]))
+        if rank == 0:
+            dump_outputs(args.dump_outputs, *last_step)
     if rank == 0:
         peak, peak_src = measured_peaks()
         traffic = ncu_traffic()
@@ -508,6 +517,24 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, res, ts):
+    """The window results the last timed step handed back (all ranks), in (key, window id) order, as DIR/window_<field>.npy in
+    float64 (exact: keys, ids, integer sums and timestamps stay below 2^53). Beyond DUMP_MAX_BYTES a fixed, seeded sample of
+    rows is written. The inputs depend only on the arguments, so two builds can be compared file by file."""
+    order = np.lexsort((res["id"], res["key"]))
+    cols = {"key": res["key"][order], "id": res["id"][order], "isum": res["isum"][order], "fsum": res["fsum"][order], "ts": ts[order]}
+    rows = DUMP_MAX_BYTES // (8 * len(cols))
+    if len(order) > rows:
+        keep = np.sort(np.random.default_rng(0).choice(len(order), rows, replace=False))
+        cols = {k: v[keep] for k, v in cols.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, v in cols.items():
+        np.save(os.path.join(path, f"window_{k}.npy"), v.astype(np.float64))
 
 
 def run_check(torch, dist, ops, ff, pipe, step, hist, out, out_ts, n_out, nb, rank, world, dev, delayed):
@@ -755,6 +782,7 @@ def main():
     ap.add_argument("--prime-steps", type=int, default=-1, help="override state priming (ncu runs); default: steady state")
     ap.add_argument("--no-check", action="store_true", help="skip the result check of the sampled keys")
     ap.add_argument("--no-extras", action="store_true", help="skip the gpu_reference and facade legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the window results of the last timed step to DIR/window_<field>.npy")
     args = ap.parse_args()
     args.warmup = max(3, args.warmup)
     if args.impl == "reference":

@@ -6,6 +6,7 @@ compiled unmodified by oracle/Makefile). Only tests/, __graft_entry__.smoke() an
 --impl reference legs may import this module; windflow_b200/ never does.
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -418,6 +419,45 @@ def sort_results(res, ts=None):
     """Canonical order for comparing window results: (key, gwid)."""
     order = np.lexsort((res["id"], res["key"]))
     return (res[order], ts[order]) if ts is not None else res[order]
+
+
+# ---------------------------------------------------------------------------------------------------
+# golden records of the reference's outputs (tests/golden/ref/*.npz, written by tests/golden/make_ref_golden.py)
+# ---------------------------------------------------------------------------------------------------
+GOLDEN_SAMPLE = 1024  # floating-point sums stored per record: all of them up to this many rows, a seeded sample beyond
+
+
+def digest(*cols):
+    """SHA-256 of the columns' bytes: a golden record keeps it in place of outputs that are compared bit for bit."""
+    h = hashlib.sha256()
+    for c in cols:
+        h.update(np.ascontiguousarray(c).tobytes())
+    return h.hexdigest()
+
+
+def _exact_cols(r, with_ts):
+    cols = [r["key"].astype("<u8"), r["id"].astype("<u8"), r["isum"].astype("<i8")]
+    return cols + [r["ts"].astype("<u8")] if with_ts else cols
+
+
+def windows_record(res, prefix, with_ts=True):
+    """Golden record of window results (fields key, id, isum, fsum[, ts]) in (key, id) order: the row count, a digest of
+    the exact columns and the floating-point sums (a fixed sample of GOLDEN_SAMPLE rows beyond that size), as npz entries."""
+    r = np.sort(res, order=["key", "id"])
+    n = len(r)
+    idx = np.arange(n) if n <= GOLDEN_SAMPLE else np.sort(np.random.default_rng(0).choice(n, GOLDEN_SAMPLE, replace=False))
+    return {prefix + ".n": np.int64(n), prefix + ".digest": np.array(digest(*_exact_cols(r, with_ts))),
+            prefix + ".idx": idx.astype("<u4"), prefix + ".fsum": r["fsum"][idx]}
+
+
+def check_windows_record(got, golden, prefix, rtol, with_ts=True):
+    """`got` equals the recorded windows: same count, same keys / window ids / integer sums (/ timestamps), floating-point
+    sums within `rtol` of the recorded ones."""
+    r = np.sort(got, order=["key", "id"])
+    assert len(r) == int(golden[prefix + ".n"]), (len(r), int(golden[prefix + ".n"]))
+    assert digest(*_exact_cols(r, with_ts)) == str(golden[prefix + ".digest"]), "keys, window ids, integer sums or timestamps differ"
+    idx = golden[prefix + ".idx"]
+    assert np.allclose(r["fsum"][idx], golden[prefix + ".fsum"], rtol=rtol, atol=0)
 
 
 # ---------------------------------------------------------------------------------------------------

@@ -1,5 +1,5 @@
 """GPU parity tests (-m gpu): Ffat_Windows_GPU (count-based) through the C ABI against the oracle, the golden
-vectors generated from the reference's wf/flatfat.hpp, and the reference's own wf/flatfat_gpu.hpp run on this GPU.
+vectors generated from the reference's wf/flatfat.hpp, and the outputs of the reference's own wf/flatfat_gpu.hpp on a B200.
 Bit-exact on keys, window ids, integer aggregates and result timestamps; floating-point aggregates within 1e-6
 relative (the pane/tree association differs from the reference's)."""
 import glob
@@ -195,16 +195,12 @@ def test_ffat_wfwin24_reference_functors(wfb, oracle):
     _check(O, got, gts, np.concatenate(exp), np.concatenate(ets), res_is32=False)
 
 
-@pytest.mark.parametrize("geom", [(64, 16, 5), (4096, 64, 1), (4096, 64, 65), (16, 4, 5)])
-def test_reference_flatfat_gpu_on_this_box(wfb, oracle, geom):
-    """The reference's own FlatFAT_GPU (wf/flatfat_gpu.hpp compiled for sm_100a into oracle/_ref) run on this GPU:
-    pins the oracle's restatement of K12-K14 and our kernels against the reference itself (power-of-two B)."""
-    import ctypes as C
-    import torch
-    O, ops = oracle, wfb
-    L = O.ref_gpu_lib()
-    if L is None:
-        pytest.skip("oracle/_ref/libwfref_flatfat_gpu.so not present")
+REF_GPU_GEOMS = [(64, 16, 5), (4096, 64, 1), (4096, 64, 65), (16, 4, 5)]  # win, slide, nb
+REF_GPU_STEP = 1000
+
+
+def ref_gpu_stream(O, geom):
+    """The stream of test_reference_flatfat_gpu_on_this_box: one key, power-of-two B, fed in chunks of REF_GPU_STEP."""
     win, slide, nb = geom
     B = (nb - 1) * slide + win
     assert B & (B - 1) == 0
@@ -214,35 +210,45 @@ def test_reference_flatfat_gpu_on_this_box(wfb, oracle, geom):
     res["key"] = 42
     res["isum"] = rng.integers(-1000, 1000, n)
     res["fsum"] = rng.random(n)
-    h = L.wfref_ffat_gpu_create(win, slide, nb, 42)
+    return res
+
+
+@pytest.mark.parametrize("geom", REF_GPU_GEOMS)
+def test_reference_flatfat_gpu_on_this_box(wfb, oracle, geom):
+    """The reference's own FlatFAT_GPU (wf/flatfat_gpu.hpp compiled for sm_100a into oracle/_ref, run on a B200; its outputs
+    on this stream are stored in tests/golden/ref/flatfat_gpu.npz): pins the oracle's restatement of K12-K14 bit for bit,
+    and through it our kernels, against the reference itself (power-of-two B)."""
+    import torch
+    O, ops = oracle, wfb
+    win, slide, nb = geom
+    res = ref_gpu_stream(O, geom)
+    n = len(res)
+    g, tag = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref", "flatfat_gpu.npz")), "_".join(map(str, geom))
+    assert O.digest(res) == str(g[tag + ".input"]), "the seeded input stream changed: the recorded outputs no longer apply"
     go = O.FfatGpuOracle(win, slide, nb)
     t = np.zeros(n, dtype=ops.TUPLE64)
     t["key"], t["ivalue"], t["fvalue"] = res["key"], res["isum"], res["fsum"]
     ff = ops.FfatWindowsGPU(ops.PROG_TUPLE64, win, slide, nb, max_keys=4)
-    step = 1000
-    ours, ours_ts = [], []
+    step = REF_GPU_STEP
+    exp, exp_ts, counts = [], [], []
     for b in range(0, n, step):
         chunk = res[b:b + step]
-        d = ops.to_device(chunk)
-        cap = (len(chunk) // slide + 2) * nb + nb
-        out = np.zeros(cap, dtype=O.RES); ots = np.zeros(cap, dtype=np.uint64)
-        k = L.wfref_ffat_gpu_process(h, C.c_void_p(d.data_ptr()), len(chunk), b, out.ctypes.data_as(C.c_void_p),
-                                     ots.ctypes.data_as(C.c_void_p), cap)
         e, et = go.process_batch(chunk, b)
-        assert k == len(e)
-        assert out[:k].tobytes() == e.tobytes()      # oracle == reference kernels, bit for bit (same tree order)
-        assert np.array_equal(ots[:k], et)
+        exp.append(e); exp_ts.append(et); counts.append(len(e))
         o, o_ts, n_out = ff.process([ops.DeviceBatch.from_host(t[b:b + step], np.arange(b, b + len(chunk), dtype=np.uint64), watermark=b)])
         torch.cuda.synchronize()
         r, rt = ff.results_to_host(o, o_ts, n_out)
-        ours.append(r); ours_ts.append(rt)
+        k = len(e)
         assert len(r) == k
         if k:
             rs, rts = O.sort_results(r, rt)
-            assert np.array_equal(rs["id"], out[:k]["id"]) and np.array_equal(rs["isum"], out[:k]["isum"])
-            assert np.allclose(rs["fsum"], out[:k]["fsum"], rtol=FP_RTOL, atol=0)
-            assert np.array_equal(rts, ots[:k])
-    L.wfref_ffat_gpu_destroy(h)
+            assert np.array_equal(rs["id"], e["id"]) and np.array_equal(rs["isum"], e["isum"])
+            assert np.allclose(rs["fsum"], e["fsum"], rtol=FP_RTOL, atol=0)
+            assert np.array_equal(rts, et)
+    # oracle == reference kernels, bit for bit (same tree order): per-chunk counts, windows and their timestamps
+    assert np.array_equal(np.array(counts, dtype=np.int64), g[tag + ".counts"])
+    assert O.digest(np.concatenate(exp)) == str(g[tag + ".out"])
+    assert O.digest(np.concatenate(exp_ts)) == str(g[tag + ".ts"])
 
 
 def test_ffat_capacity_error_flag(wfb, oracle):

@@ -1,6 +1,6 @@
 """CPU tests (-m "not gpu"): the oracle against the golden vectors generated from the reference's own
-wf/flatfat.hpp (tests/golden/*.npz), against the live reference pin when oracle/_ref is present, and its own
-internal consistency (tree order vs linear fold, GPU-operator semantics vs CPU-operator windows)."""
+wf/flatfat.hpp (tests/golden/*.npz, tests/golden/ref/flatfat_cpu.npz), and its own internal consistency
+(tree order vs linear fold, GPU-operator semantics vs CPU-operator windows)."""
 import glob
 import os
 
@@ -76,22 +76,40 @@ def test_gpu_operator_oracle_matches_reference_golden(oracle, path, nb):
     assert len(out) == exp
 
 
-def test_cpu_ffat_matches_live_reference(oracle):
-    O = oracle
-    if O.ref_cpu_lib() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
+LIVE_CASES = [(4, 2, 3), (8, 8, 1), (10, 3, 5), (7, 7, 2), (5, 1, 4), (32, 8, 6), (256, 64, 3)]  # win, slide, nkeys
+
+
+def live_streams(O):
+    """The streams of test_cpu_ffat_matches_live_reference, one per LIVE_CASES entry, all drawn from one seeded generator."""
     rng = np.random.default_rng(7)
-    for (W, S, nk) in [(4, 2, 3), (8, 8, 1), (10, 3, 5), (7, 7, 2), (5, 1, 4), (32, 8, 6), (256, 64, 3)]:
-        n = max(6000, W * nk * 6)
-        r = _stream(O, rng, n, nk)
-        oc, rc = O.FfatCpuOracle(W, S), O.RefFfatCpu(W, S)
-        for b in range(0, n, 257):
-            o, ot = oc.process(r[b:b + 257], b)
-            q, qt = rc.process(r[b:b + 257], b)
-            assert np.array_equal(ot, qt)
-            assert o.tobytes() == q.tobytes()
-        eo, _ = oc.eos(); er, _ = rc.eos()
-        assert O.sort_results(eo).tobytes() == O.sort_results(er).tobytes()
+    for (W, S, nk) in LIVE_CASES:
+        yield W, S, nk, _stream(O, rng, max(6000, W * nk * 6), nk)
+
+
+def ffat_cpu_record(O, ffat, r):
+    """Digests of what a CPU FlatFAT operator emits on stream r in batches of 257 (windows, their timestamps, the windows
+    flushed at end of stream) and the per-batch window counts."""
+    outs, tss, counts = [], [], []
+    for b in range(0, len(r), 257):
+        o, ot = ffat.process(r[b:b + 257], b)
+        outs.append(o); tss.append(ot); counts.append(len(o))
+    eo, _ = ffat.eos()
+    return {"out": O.digest(np.concatenate(outs)), "ts": O.digest(np.concatenate(tss)), "eos": O.digest(O.sort_results(eo)),
+            "counts": np.array(counts, dtype=np.int64)}
+
+
+def test_cpu_ffat_matches_live_reference(oracle):
+    """The oracle's CPU FlatFAT operator equals, bit for bit, the reference's own wf/flatfat.hpp under the restated replica
+    loop (oracle/_ref/libwfref_flatfat.so), whose outputs on these streams are stored in tests/golden/ref/flatfat_cpu.npz."""
+    O = oracle
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref", "flatfat_cpu.npz"))
+    for W, S, nk, r in live_streams(O):
+        t = f"{W}_{S}_{nk}"
+        assert O.digest(r) == str(g[t + ".input"]), "the seeded input stream changed: the recorded outputs no longer apply"
+        got = ffat_cpu_record(O, O.FfatCpuOracle(W, S), r)
+        assert np.array_equal(got["counts"], g[t + ".counts"])
+        for k in ("out", "ts", "eos"):
+            assert got[k] == str(g[t + "." + k]), (t, k)
 
 
 def test_stream_generator(oracle):

@@ -1,28 +1,31 @@
-"""The oracle and the CUDA path against the UNMODIFIED reference running live.
+"""The oracle and the CUDA path against what the UNMODIFIED reference computed on the same inputs.
 
 oracle/_ref/ref_pipeline_{cpu,gpu} are the reference's own wf/windflow.hpp / wf/windflow_gpu.hpp (PipeGraph, MultiPipe, emitters,
-collectors, Map/Filter/Ffat_Windows and their *_GPU versions) compiled from /root/reference by oracle/Makefile over this
-repository's FastFlow-compatible runtime (include/ff/) and driven by oracle/ref_pipeline.cu on the bench schema.
+collectors, Map/Filter/Ffat_Windows and their *_GPU versions) compiled from the reference sources by oracle/Makefile over this
+repository's FastFlow-compatible runtime (include/ff/) and driven by oracle/ref_pipeline.cu on the bench schema. Their outputs
+on the inputs below are stored under tests/golden/ref/ (tests/golden/make_ref_golden.py), so the tests need no reference build.
 
-  CPU (here):    reference CPU pipeline Source -> Map -> Filter -> Ffat_Windows(CB), 4 replicas  ==  the oracle's restatement
-  GPU (the box): reference GPU pipeline Source -> Map_GPU -> Filter_GPU -> Ffat_Windows_GPU, count-based AND time-based
-                 ==  the oracle's restatement  ==  libwfb200's kernels (through the C ABI)
-                 reference Map_GPU -> Filter_GPU and Reduce_GPU == oracle == kernels
+  CPU:  reference CPU pipeline Source -> Map -> Filter -> Ffat_Windows(CB), 4 replicas  ==  the oracle's restatement
+  GPU:  reference GPU pipeline Source -> Map_GPU -> Filter_GPU -> Ffat_Windows_GPU, count-based AND time-based
+        ==  the oracle's restatement  ==  libwfb200's kernels (through the C ABI)
+        reference Map_GPU -> Filter_GPU and Reduce_GPU == oracle == kernels
 This is what pins the oracle's trigger loops (count-based groups, time-based panes / watermarks / lateness, reduce, compaction),
 not only the FlatFAT they share: SURVEY.md 8c.
 """
-import json
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_CPU = os.path.join(ROOT, "oracle", "_ref", "ref_pipeline_cpu")
-REF_GPU = os.path.join(ROOT, "oracle", "_ref", "ref_pipeline_gpu")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "ref")
+CPU_CASES = [(7, 64, 16), (100, 1024, 32), (5, 10, 3)]                                          # nkeys, win, slide
+CB_CASES = [(13, 64, 16, 2, 2048), (5, 1024, 32, 9, 4096), (64, 4096, 64, 65, 65536), (3, 10, 3, 4, 1000)]  # nkeys, win, slide, nb, batch
+TB_CASES = [("monotone", 7, 4000, 1000, 3, 0), ("ooo", 11, 3000, 500, 4, 400), ("gaps", 5, 2000, 2000, 2, 0),
+            ("ooo", 4, 900, 300, 5, 0)]                                                          # kind, nkeys, win, slide, nb, lateness
+MF_BATCH, MF_N, MF_KEYS = 4096, 4096 * 6 + 123, 300
+TB_BATCH, TB_N = 2048, 2048 * 14 + 700
 RES_TS = np.dtype([("key", "<u8"), ("id", "<u8"), ("isum", "<i8"), ("fsum", "<f8"), ("ts", "<u8")])
-TUP_TS = np.dtype([("key", "<u8"), ("id", "<u8"), ("ivalue", "<i8"), ("fvalue", "<f8"), ("pad", "<u8", (4,)), ("ts", "<u8")])
 
 
 def batch_watermarks(ts, batch):
@@ -35,39 +38,31 @@ def batch_watermarks(ts, batch):
     return wm
 
 
-def write_stream(path, tuples, ts, wm):
-    with open(path, "wb") as f:
-        f.write(np.uint64(len(tuples)).tobytes())
-        f.write(np.ascontiguousarray(tuples).tobytes()); f.write(np.ascontiguousarray(ts, dtype=np.uint64).tobytes())
-        f.write(np.ascontiguousarray(wm, dtype=np.uint64).tobytes())
+def mf_digest(tuples, ts):
+    """Digest of the Map -> Filter output columns in stream order (the golden record of ref_pipeline_gpu gpu_mf)."""
+    from oracle import oracle as O
+    return O.digest(tuples["key"].astype("<u8"), tuples["id"].astype("<u8"), tuples["ivalue"].astype("<i8"),
+                    tuples["fvalue"].astype("<f8"), np.asarray(ts).astype("<u8"))
 
 
-def run_ref(exe, mode, tmp_path, tuples, ts, wm, dtype=RES_TS, **kw):
-    inp, out = str(tmp_path / "in.bin"), str(tmp_path / f"{mode}.out")
-    write_stream(inp, tuples, ts, wm)
-    args = [exe, mode, f"in={inp}", f"out={out}"] + [f"{k}={v}" for k, v in kw.items()]
-    p = subprocess.run(args, capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0, p.stdout[-2000:] + p.stderr[-2000:]
-    info = json.loads(p.stdout.strip().splitlines()[-1])
-    raw = open(out, "rb").read()
-    m = int(np.frombuffer(raw[:8], dtype=np.uint64)[0])
-    res = np.frombuffer(raw[8:], dtype=dtype, count=m)
-    assert info["results"] == m
-    return res, info
+def tag(case):
+    return "_".join(str(x) for x in case)
 
 
-def sort_rows(a, with_ts=True):
-    return np.sort(a, order=["key", "id"])
+def golden(name):
+    return np.load(os.path.join(GOLDEN, name + ".npz"))
 
 
-def assert_windows_equal(got, exp, check_ts=True, rtol=1e-9):
-    assert len(got) == len(exp), (len(got), len(exp))
-    g, e = np.sort(got, order=["key", "id"]), np.sort(exp, order=["key", "id"])
-    assert np.array_equal(g["key"], e["key"]) and np.array_equal(g["id"], e["id"])
-    assert np.array_equal(g["isum"], e["isum"])
-    assert np.allclose(g["fsum"], e["fsum"], rtol=rtol, atol=0)
-    if check_ts:
-        assert np.array_equal(g["ts"], e["ts"])
+def cpu_stream(O, nkeys):
+    return O.gen_tuple64(0, 200_000, O.KEY_UNIFORM, nkeys)
+
+
+def cb_stream(O, nkeys, win, batch):
+    n = batch * 12 + batch // 3  # a ragged last batch too
+    if win == 4096:
+        n = batch * 20
+    tuples, ts = O.gen_tuple64(0, n, O.KEY_UNIFORM, nkeys)
+    return tuples, ts, batch_watermarks(ts, batch)
 
 
 def with_ts(res, ts):
@@ -79,22 +74,21 @@ def with_ts(res, ts):
 
 
 # ---- CPU: the reference's Map -> Filter -> Ffat_Windows pipeline == the oracle's restatement -------------------------------------
-@pytest.mark.skipif(not os.path.isdir("/root/reference/wf"), reason="the reference is only present in the build container")
-@pytest.mark.parametrize("nkeys,win,slide", [(7, 64, 16), (100, 1024, 32), (5, 10, 3)])
-def test_reference_cpu_pipeline_matches_oracle(oracle, tmp_path, nkeys, win, slide):
-    subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s", REF_CPU])
+@pytest.mark.parametrize("nkeys,win,slide", CPU_CASES)
+def test_reference_cpu_pipeline_matches_oracle(oracle, nkeys, win, slide):
+    """Reference run: ref_pipeline_cpu cpu_cb, par=4 (1 source + 4 map/filter + 4 ffat + 1 sink: cfg 1 of BASELINE.json), det=1,
+    watermarks every 4096 tuples."""
     O = oracle
-    n = 200_000
-    tuples, ts = O.gen_tuple64(0, n, O.KEY_UNIFORM, nkeys)
-    ref, info = run_ref(REF_CPU, "cpu_cb", tmp_path, tuples, ts, batch_watermarks(ts, 4096), keys=nkeys, win=win, slide=slide, par=4, det=1)
-    assert info["threads"] >= 10  # 1 source + 4 map/filter + 4 ffat + 1 sink (cfg 1 of BASELINE.json)
+    tuples, ts = cpu_stream(O, nkeys)
     surv, sts, _ = O.map_filter_tuple64(tuples, ts, 1, 2, 1.0000001, 1)
     cpu = O.FfatCpuOracle(win, slide)
     r, rt = cpu.process(O.lift_tuple64(surv), 0)
     r2, rt2 = cpu.eos()   # the CPU operator flushes the partial windows at end of stream (wf/ffat_replica.hpp:406-427)
     exp = with_ts(np.concatenate([r, r2]), np.concatenate([rt, rt2]))
-    assert len(ref) > 0
-    assert_windows_equal(ref, exp, check_ts=False)  # (the CPU operator's result timestamps depend on replica interleaving)
+    g = golden("cpu_pipeline")
+    assert int(g[tag((nkeys, win, slide)) + ".n"]) > 0
+    # (the CPU operator's result timestamps depend on replica interleaving: not compared)
+    O.check_windows_record(exp, g, tag((nkeys, win, slide)), rtol=1e-9, with_ts=False)
 
 
 # ---- GPU: reference GPU operators == oracle == libwfb200 ----------------------------------------------------------------------------
@@ -124,22 +118,16 @@ def _oracle_cb(O, tuples, ts, wm, batch, win, slide, nb):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("nkeys,win,slide,nb,batch", [(13, 64, 16, 2, 2048), (5, 1024, 32, 9, 4096), (64, 4096, 64, 65, 65536), (3, 10, 3, 4, 1000)])
-def test_reference_gpu_cb_pipeline_matches_oracle_and_kernels(oracle, wfb, tmp_path, nkeys, win, slide, nb, batch):
-    if not os.path.exists(REF_GPU):
-        pytest.skip("oracle/_ref/ref_pipeline_gpu was not built (needs /root/reference at build time)")
+@pytest.mark.parametrize("nkeys,win,slide,nb,batch", CB_CASES)
+def test_reference_gpu_cb_pipeline_matches_oracle_and_kernels(oracle, wfb, nkeys, win, slide, nb, batch):
     O = oracle
-    n = batch * 12 + batch // 3  # a ragged last batch too
-    if win == 4096:
-        n = batch * 20
-    tuples, ts = O.gen_tuple64(0, n, O.KEY_UNIFORM, nkeys)
-    wm = batch_watermarks(ts, batch)
-    ref, _ = run_ref(REF_GPU, "gpu_cb", tmp_path, tuples, ts, wm, keys=nkeys, win=win, slide=slide, nb=nb, batch=batch)
+    tuples, ts, wm = cb_stream(O, nkeys, win, batch)
+    g, t = golden("gpu_cb"), tag((nkeys, win, slide, nb, batch))
+    assert int(g[t + ".n"]) > 0
     exp = _oracle_cb(O, tuples, ts, wm, batch, win, slide, nb)
-    assert len(ref) > 0
-    assert_windows_equal(ref, exp, rtol=1e-9)            # oracle == reference (same tree association: tight)
+    O.check_windows_record(exp, g, t, rtol=1e-9)         # oracle == reference (same tree association: tight)
     got = _ours_cb(wfb, tuples, ts, wm, batch, win, slide, nb, nkeys)
-    assert_windows_equal(got, ref, rtol=1e-6)            # kernels == reference (pane-then-tree association: north_star's 1e-6)
+    O.check_windows_record(got, g, t, rtol=1e-6)         # kernels == reference (pane-then-tree association: north_star's 1e-6)
 
 
 def _tb_stream(O, n, nkeys, kind, seed=3):
@@ -158,18 +146,14 @@ def _tb_stream(O, n, nkeys, kind, seed=3):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("kind,nkeys,win,slide,nb,lateness", [("monotone", 7, 4000, 1000, 3, 0), ("ooo", 11, 3000, 500, 4, 400), ("gaps", 5, 2000, 2000, 2, 0),
-                                                           ("ooo", 4, 900, 300, 5, 0)])
-def test_reference_gpu_tb_pipeline_matches_oracle_and_kernels(oracle, wfb, tmp_path, kind, nkeys, win, slide, nb, lateness):
-    """Time-based windows: the reference's own Ffat_Replica_GPU::process_batch_tb / process_wins_tb / PendingPanes_Queue, live."""
-    if not os.path.exists(REF_GPU):
-        pytest.skip("oracle/_ref/ref_pipeline_gpu was not built (needs /root/reference at build time)")
+@pytest.mark.parametrize("kind,nkeys,win,slide,nb,lateness", TB_CASES)
+def test_reference_gpu_tb_pipeline_matches_oracle_and_kernels(oracle, wfb, kind, nkeys, win, slide, nb, lateness):
+    """Time-based windows: the reference's own Ffat_Replica_GPU::process_batch_tb / process_wins_tb / PendingPanes_Queue."""
     import torch
     O, ops = oracle, wfb
-    batch, n = 2048, 2048 * 14 + 700
+    batch, n = TB_BATCH, TB_N
     tuples, ts = _tb_stream(O, n, nkeys, kind)
     wm = batch_watermarks(ts, batch)
-    ref, _ = run_ref(REF_GPU, "gpu_tb", tmp_path, tuples, ts, wm, keys=nkeys, win=win, slide=slide, nb=nb, batch=batch, lateness=lateness)
     to = O.FfatTbOracle(win, slide, lateness, nb)
     f = ops.functors(map_kind=1, iadd=2, fscale=1.0000001, filt_kind=1)
     ff = ops.FfatWindowsGPU(ops.PROG_TUPLE64, win, slide, nb, max_keys=64, win_type=1, lateness=lateness)
@@ -185,27 +169,23 @@ def test_reference_gpu_tb_pipeline_matches_oracle_and_kernels(oracle, wfb, tmp_p
         got_r.append(r); got_t.append(t)
     exp = with_ts(np.concatenate(exp_r), np.concatenate(exp_t))
     got = with_ts(np.concatenate(got_r), np.concatenate(got_t))
-    assert len(ref) > 0
-    assert_windows_equal(exp, ref, rtol=1e-6)    # the oracle's restatement == the reference (pins SURVEY.md row a10)
-    assert_windows_equal(got, ref, rtol=1e-6)    # kernels == the reference
+    g, t = golden("gpu_tb"), tag((kind, nkeys, win, slide, nb, lateness))
+    assert int(g[t + ".n"]) > 0
+    O.check_windows_record(exp, g, t, rtol=1e-6)    # the oracle's restatement == the reference (pins SURVEY.md row a10)
+    O.check_windows_record(got, g, t, rtol=1e-6)    # kernels == the reference
 
 
 @pytest.mark.gpu
-def test_reference_gpu_map_filter_and_reduce_match_oracle_and_kernels(oracle, wfb, tmp_path):
-    if not os.path.exists(REF_GPU):
-        pytest.skip("oracle/_ref/ref_pipeline_gpu was not built (needs /root/reference at build time)")
+def test_reference_gpu_map_filter_and_reduce_match_oracle_and_kernels(oracle, wfb):
     import torch
     O, ops = oracle, wfb
-    batch, n, nkeys = 4096, 4096 * 6 + 123, 300
+    batch, n, nkeys = MF_BATCH, MF_N, MF_KEYS
     tuples, ts = O.gen_tuple64(0, n, O.KEY_UNIFORM, nkeys)
-    wm = batch_watermarks(ts, batch)
+    g = golden("gpu_mf_red")
     # Map_GPU -> Filter_GPU: the stream of survivors, in order (one source, one replica each)
-    ref, _ = run_ref(REF_GPU, "gpu_mf", tmp_path, tuples, ts, wm, dtype=TUP_TS, batch=batch)
     surv, sts, _ = O.map_filter_tuple64(tuples, ts, 1, 2, 1.0000001, 1)
-    assert len(ref) == len(surv)
-    for fld in ("key", "id", "ivalue"):
-        assert np.array_equal(ref[fld], surv[fld])
-    assert np.array_equal(ref["fvalue"], surv["fvalue"]) and np.array_equal(ref["ts"], sts)
+    assert len(surv) == int(g["mf.n"])
+    assert mf_digest(surv, sts) == str(g["mf.digest"])   # key, id, ivalue, fvalue and ts of every survivor, bit for bit
     eng = ops.Engine(ops.PROG_TUPLE64)
     f = ops.functors(map_kind=1, iadd=2, fscale=1.0000001, filt_kind=1)
     got = []
@@ -217,12 +197,11 @@ def test_reference_gpu_map_filter_and_reduce_match_oracle_and_kernels(oracle, wf
     got = np.concatenate(got)
     assert got.tobytes() == np.ascontiguousarray(surv).tobytes()
     # Reduce_GPU keyed: one item per distinct key and batch, ascending key
-    ref, _ = run_ref(REF_GPU, "gpu_red", tmp_path, tuples, ts, wm, dtype=TUP_TS, batch=batch)
     exp = []
     for i in range(0, n, batch):
         r, rt = O.reduce_tuple64(tuples[i:i + batch], ts[i:i + batch])
         exp.append(r)
     exp = np.concatenate(exp)
-    assert len(ref) == len(exp)
-    assert np.array_equal(ref["key"], exp["key"]) and np.array_equal(ref["ivalue"], exp["ivalue"])
-    assert np.allclose(ref["fvalue"], exp["fvalue"], rtol=1e-9)
+    assert len(exp) == int(g["red.n"])
+    assert O.digest(exp["key"].astype("<u8"), exp["ivalue"].astype("<i8")) == str(g["red.digest"])
+    assert np.allclose(g["red.fvalue"], exp["fvalue"], rtol=1e-9)
